@@ -22,9 +22,13 @@ Printed JSON (one line, rank 0): the driver contract plus
   stock_torch_gpu the same oracle port (the op sequence the reference launches) on THIS GPU, fp32 and TF32
   cfg4_stream     config 4's data path: fp16 chunks from disk -> pinned -> HBM -> device-side gather -> step, with
                   the end-of-chunk metric gather (also a workload of its own: --workload cfg4_stream)
+
+--dump-outputs DIR writes what the last step of the `value` loop returned, and the parameters it left, as .npy files
+(see dump_outputs); the inputs depend only on the arguments, so two builds can be compared file by file.
 """
 import argparse
 import json
+import math
 import os
 import shutil
 import subprocess
@@ -83,6 +87,15 @@ def synth_batches(n_batches, B, d, seed, pin=False):
     return out
 
 
+def _die_with_parent():
+    """Runs in the sampler's child before exec: the kernel sends it SIGTERM when bench.py exits, also on an exception
+    or a kill, so a failed run leaves no sampling nvidia-smi behind."""
+    import ctypes
+    import signal
+    PR_SET_PDEATHSIG = 1
+    ctypes.CDLL(None).prctl(PR_SET_PDEATHSIG, signal.SIGTERM)
+
+
 class ClockSampler:
     QUERY = ("timestamp,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,"
              "clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown,"
@@ -99,7 +112,8 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.gpu), f"--query-gpu={self.QUERY}",
                                           "--format=csv,noheader,nounits", "-lms", "10"],
-                                         stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
+                                         stdout=open(self.path, "w"), stderr=subprocess.DEVNULL,
+                                         preexec_fn=_die_with_parent)
         except OSError:
             self.proc = None
 
@@ -190,6 +204,39 @@ def ncu_traffic():
     """DRAM bytes per launch of every kernel of a step from the committed `ncu --set full` capture (profiles/)."""
     path = os.path.join(ROOT, "profiles", "ncu_traffic.json")
     return json.load(open(path)) if os.path.exists(path) else None
+
+
+DUMP_BYTES = 60_000_000                 # with the .npy headers, under 64 MB in all
+
+
+def dump_outputs(folder, enss, results):
+    """Writes, as float32 ``folder/<name>.npy``, what one step returned to its caller — every loss term [M], the mean
+    L0 [M] and the code [M, B, n] of ``aux["c"]`` — and every parameter the step left ([M, n, d] / [M, n]); names
+    carry a ``g<i>_`` prefix when the workload steps several ensembles. An array larger than its share of
+    DUMP_BYTES is cut along axis 1 (batch rows of the code, dictionary rows of a parameter) to a seeded, sorted subset
+    of indices, the same on every run. Returns {name: shape written}."""
+    arrays = {}
+    for g, (e, (losses, aux)) in enumerate(zip(enss, results)):
+        pre = f"g{g}_" if len(enss) > 1 else ""
+        arrays.update({pre + k: v for k, v in losses.items()})
+        arrays[pre + "mean_l0"] = aux["c"].count_nonzero(dim=-1).float().mean(dim=-1)
+        arrays[pre + "code"] = aux["c"]                       # CodeProxy: read back from the engine when indexed
+        arrays.update({pre + k: v for k, v in e.params.items()})
+    os.makedirs(folder, exist_ok=True)
+    budget, left, shapes = DUMP_BYTES, len(arrays), {}
+    for name, v in sorted(arrays.items(), key=lambda kv: math.prod(kv[1].shape)):
+        share = budget // left                                # small arrays leave their unused share to the large
+        left -= 1
+        size = 4 * math.prod(v.shape)
+        if size > share:
+            keep = max(1, share // (size // v.shape[1]))
+            idx = torch.randperm(v.shape[1], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            v = v[:, idx.to(v.device)]
+        a = v.float().cpu().numpy()
+        np.save(os.path.join(folder, name + ".npy"), a)
+        budget -= a.nbytes
+        shapes[name] = list(a.shape)
+    return shapes
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -484,7 +531,13 @@ def main():
     ap.add_argument("--stream-rows", type=int, default=1 << 21, help="rows per streamed chunk (reference: 2^21 at d=512)")
     ap.add_argument("--feed", default="per_rank", choices=["per_rank", "broadcast", "both"],
                     help="cfg4_stream: every rank reads/copies its own chunk, or rank 0 reads and NCCL broadcasts")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs and parameters to DIR/<name>.npy (rank 0, engine only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs writes the engine's outputs: use it with --impl engine")
     global ACT_FP16
     ACT_FP16 = args.act_precision == "fp16"
 
@@ -542,10 +595,8 @@ def main():
         torch.cuda.synchronize()
 
     def step_all(x):
-        r = None
-        for e in enss:
-            r = e.step_batch(x)
-        return r
+        """(losses, aux) of every ensemble, in order."""
+        return [e.step_batch(x) for e in enss]
 
     # ---------------- device-resident run: `value` (nothing but step_batch calls between the two events)
     windows = {}
@@ -557,14 +608,18 @@ def main():
     t_begin = time.time()
     e0.record()
     for i in range(K):
-        losses, aux = step_all(pool[i % n_pool])
+        results = step_all(pool[i % n_pool])
     e1.record()
     barrier()
     windows["value"] = (t_begin, time.time())
     ms = e0.elapsed_time(e1)
     launches = K * sum(e.gpu_launches_last_call() for e in enss)
-    final_loss = losses["loss"].detach().clone()
+    final_loss = results[-1][0]["loss"].detach().clone()
     arith_resolved = ens.resolved_arith()
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = dump_outputs(args.dump_outputs, enss, results)
+    del results
 
     # ---------------- per-phase device times: a separate short loop with libsce's events switched on
     for e in enss:
@@ -597,7 +652,7 @@ def main():
                 a.record()
                 x = x.to(dev, non_blocking=True)                          # pinned host -> device on the compute stream
                 b.record()
-            losses, aux = step_all(x)
+            losses, aux = step_all(x)[-1]
             if not prefetch and i >= 2:
                 c.record()
                 evs.append((a, b, c))
@@ -729,6 +784,10 @@ def main():
             "gemms": gemms,
             "final_loss_mean": float(final_loss.mean()),
         }
+        if dumped is not None:
+            line["dump_outputs"] = {"dir": args.dump_outputs, "shapes": dumped,
+                                    "what": f"step {W + K} (the last of `value`); axis 1 sampled where an array "
+                                            "exceeds its share of 60 MB"}
         tr = (ncu_traffic() or {}).get(arith)
         if tr and args.workload == "cfg2":
             line["roofline"]["traffic"] = tr["dw_dram_bytes_per_launch"]
