@@ -92,7 +92,9 @@ typedef struct sce_buffers {
   const float* l1_alpha;          /* [M]   buffers["l1_alpha"]; NULL = 0 (topk) */
   const float* bias_decay;        /* [M]   buffers["bias_decay"]; NULL = 0 */
   const unsigned char* coef_mask; /* [M,n] buffers["coef_mask"] (1 = unused coefficient) or NULL */
-  const long long* sparsity;      /* [M]   buffers["sparsity"] (topk k) or NULL */
+  const long long* sparsity;      /* [M]   buffers["sparsity"] (topk k) or NULL. Every k in [1, n], and, when
+                                     desc.topk_k_max is in 1..256 (the plan keeps k-sparse lists), k <= topk_k_max;
+                                     read by sce_prepare, which rejects other values */
   void* workspace;                /* >= sce_workspace_bytes(desc), 1024-byte aligned */
   size_t workspace_bytes;
   const float* center_trans;      /* [M,d]   buffers["center_trans"]  (desc.centering != 0; else NULL) */
@@ -117,7 +119,10 @@ int sce_plan_create(const sce_desc* desc, const sce_buffers* buffers, sce_plan**
 int sce_plan_destroy(sce_plan* plan);
 
 /* (Re)derive the normalised operand planes of the dictionaries from the fp32 parameters. Must be
- * called once before the first step and again whenever the caller modified the parameters itself. */
+ * called once before the first step and again whenever the caller modified the parameters itself.
+ * SCE_TOPK: also re-reads buffers.sparsity (the k of each model) and returns SCE_ERR_INVALID if a k is < 1 or > n, or,
+ * on a plan that keeps k-sparse lists, > desc.topk_k_max: the lists hold at most that many entries per row, so a larger
+ * k needs a new plan. Until it succeeds the plan must not run. */
 int sce_prepare(sce_plan* plan, void* stream);
 
 /* One optimisation step for all M models on one batch == FunctionalEnsemble.step_batch (ensemble.py:175-193):

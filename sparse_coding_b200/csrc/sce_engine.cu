@@ -1019,6 +1019,21 @@ int sce_prepare(sce_plan* p, void* stream) {
   CUDA_TRY(cudaMemsetAsync(p->res_flags, 0, kFlagWords * sizeof(uint32_t), st));   // residual flag, input range monitor, health
   const sce_desc& d = p->d;
   const long long rows = (long long)d.n_models * d.n;
+  std::vector<long long> ks;
+  if (d.variant == SCE_TOPK) {
+    // the selection kernel takes k from buffers.sparsity as it is: k < 1 leaves its bound unset, and a plan with lists
+    // records at most its capacity of the k entries it scatters, so the next call would not clear the others
+    ks.resize(d.n_models);
+    CUDA_TRY(cudaMemcpyAsync(ks.data(), p->b.sparsity, ks.size() * sizeof(long long), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    for (int m = 0; m < d.n_models; ++m) {
+      if (ks[m] < 1 || ks[m] > d.n)
+        return fail(SCE_ERR_INVALID, "model %d: sparsity k = %lld outside [1, n = %d]", m, ks[m], d.n);
+      if (p->tk_kmax && ks[m] > d.topk_k_max)
+        return fail(SCE_ERR_INVALID, "model %d: sparsity k = %lld above the plan's topk_k_max = %d (create a new plan)", m,
+                    ks[m], d.topk_k_max);
+    }
+  }
   if (d.variant == SCE_TOPK && p->tk_kmax) {
     // the top-k selection keeps the code planes (and, in k-sparse plans, the code-gradient planes) all-zero except for
     // the entries its lists record: start them zeroed, with empty lists
@@ -1030,10 +1045,7 @@ int sce_prepare(sce_plan* p, void* stream) {
     CUDA_TRY(cudaMemsetAsync(p->dz_hi, 0, el * 4, st));   // (the code-gradient planes are one contiguous block, 4 B / element)
     CUDA_TRY(cudaMemsetAsync(p->act_pos, 0, (size_t)d.n_models * ((d.n + 31) / 32) * d.batch_max * sizeof(uint32_t), st));
     CUDA_TRY(cudaMemsetAsync(p->tk_cnt, 0, (size_t)d.n_models * d.batch_max * sizeof(int), st));
-    // k classes for the gather kernel: rows of shared memory in {8, 16, 32, 64, ...} capped at the list capacity
-    std::vector<long long> ks(d.n_models);
-    CUDA_TRY(cudaMemcpyAsync(ks.data(), p->b.sparsity, ks.size() * sizeof(long long), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
+    // k classes for the gather kernel: rows of shared memory in {16, 32, 64} and the list capacity, each capped at it
     const int caps[4] = {16, 32, 64, p->tk_kmax};
     std::vector<int> order;
     p->tk_groups = 0;
@@ -1043,8 +1055,7 @@ int sce_prepare(sce_plan* p, void* stream) {
       const int cap = caps[g] < p->tk_kmax ? caps[g] : p->tk_kmax;
       if (g > 0 && cap <= lo) continue;
       for (int m = 0; m < d.n_models; ++m) {
-        const long long k = ks[m] < 1 ? 1 : (ks[m] > p->tk_kmax ? (long long)p->tk_kmax : ks[m]);   // (kernels clip k the same way)
-        if (k > lo && k <= cap) order.push_back(m);
+        if (ks[m] > lo && ks[m] <= cap) order.push_back(m);   // (1 <= k <= topk_k_max <= tk_kmax: checked above)
       }
       p->tk_group_krows[p->tk_groups] = cap;
       p->tk_group_off[++p->tk_groups] = (int)order.size();

@@ -200,6 +200,7 @@ class FunctionalEnsemble:
         self._variant = variant
         self._plan = None
         self._plan_key = None
+        self._plan_k_max = 0              # TopK: the largest sparsity the current plan was built for
         self._ws = None
         self._centering = None
         self._serial = 0
@@ -238,8 +239,20 @@ class FunctionalEnsemble:
         return not (bool((b["center_rot"] == eye).all()) and bool((b["center_trans"] == 0).all())
                     and bool((b["center_scale"] == 1).all()))
 
+    def _topk_k_max(self) -> int:
+        """Largest ``buffers["sparsity"]`` of a TopK ensemble (0 for the other variants); raises ``ValueError`` naming
+        the model when a k is outside [1, n] (``torch.topk`` raises for k > n in the reference)."""
+        if self._variant != "topk":
+            return 0
+        ks = [int(k) for k in self.buffers["sparsity"].reshape(-1).tolist()]
+        for m, k in enumerate(ks):
+            if not 1 <= k <= self._n:
+                raise ValueError(f"model {m}: sparsity k = {k} is outside [1, n = {self._n}]")
+        return max(ks)
+
     def _build_plan(self, batch_max: int, x_per_model: bool, centering: int = 0):
         dev = self._require_cuda()
+        k_max = self._topk_k_max()
         lib = _lib.load()
         for k, v in self.params.items():
             if v.dtype != torch.float32:
@@ -256,7 +269,7 @@ class FunctionalEnsemble:
             fwd_passes=self.fwd_passes, bwd_passes=self.bwd_passes,
             norm_floor=0.0 if self._variant == "topk" else 1e-8,
             arith=_lib.ARITH_CODE[getattr(self, "_arith_fallback", None) or getattr(self, "arith", "auto")],
-            topk_k_max=int(self.buffers["sparsity"].max()) if self._variant == "topk" else 0,
+            topk_k_max=k_max,
             centering=centering)
         nbytes = lib.sce_workspace_bytes(C.byref(desc))
         if nbytes == 0:
@@ -307,6 +320,7 @@ class FunctionalEnsemble:
             self._plan = plan
             self._engine_buffers = eb
             self._plan_key = (batch_max, bool(x_per_model), int(centering))
+            self._plan_k_max = k_max
             _lib.check(lib.sce_set_step_count(plan, self._steps), "sce_set_step_count")
             _lib.check(lib.sce_prepare(plan, self._stream()), "sce_prepare")
         self._plan_steps = 0
@@ -487,9 +501,14 @@ class FunctionalEnsemble:
 
     def refresh(self):
         """Call after modifying ``params`` / ``buffers`` from outside the engine (re-derives the operand
-        copies and the cached centring check)."""
+        copies and the cached centring check). A TopK ensemble whose largest ``sparsity`` changed gets a new plan:
+        the list capacity, the gather-path choice and the slice count all follow from it."""
         self._centering = None
-        if self._plan is not None:
+        k_max = self._topk_k_max()
+        if self._plan is not None and k_max != self._plan_k_max:
+            key = self._plan_key
+            self._build_plan(key[0], key[1], key[2])
+        elif self._plan is not None:
             # engine-side copies of the buffers (dtype-converted hyper-parameter vectors, uint8 coef_mask, int64
             # sparsity) keep their addresses — the plan holds the pointers — and are refilled in place
             for name, t in (self._engine_buffers or {}).items():
